@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — accessibility nt/s of the `db` hot path on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   torchrun --nproc-per-node N ... bench.py --gpus N ...          (one rank per GPU, launched by the driver)
 
 A *step* is one pass of the hot path (inside + outside + accessibility, everything the reference's
@@ -17,6 +17,12 @@ strided sample of the dataset, outside the timed region.
 
 `--impl reference` times the reference's own CPU implementation (oracle/_ref, the unmodified raccess.cpp
 compiled with OpenMP, all host threads) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes what the last timed step computed for a fixed, seeded sample of the dataset's
+transcripts (the same sample whatever the number of ranks), so that two builds can be compared output for
+output: DIR/acc.npy and DIR/cond.npy (float32, the (acc, cond) vectors of the sampled transcripts concatenated
+in index order), DIR/transcript_index.npy (float64, the sampled transcripts' indices in the dataset) and
+DIR/lengths.npy (float64, their lengths, which split acc and cond per transcript).
 """
 from __future__ import annotations
 
@@ -36,6 +42,9 @@ DELTA = 5
 N_TRANSCRIPTS = 100_000       # cfg2 in full (BASELINE.json configs[1]); --transcripts N takes the first N of the stream
 WORKLOAD = ("cfg2: GENCODE-like synthetic transcripts, length=clip(round(LogNormal(ln1500,0.75)),200,5000), "
             "GC=0.45, W=70, delta=5")
+# --dump-outputs sample: at most 1,024 transcripts of at most 5,000 nt, i.e. <= 41 MB of float32 (acc + cond)
+DUMP_TRANSCRIPTS = 1024
+DUMP_SEED = 0
 
 
 def host_cores() -> int:
@@ -64,6 +73,24 @@ def rank_shard(seqs, rank: int, world: int):
         return list(seqs), np.arange(len(seqs))
     ids = lpt_shard([len(s) for s in seqs], world)[rank]
     return [seqs[k] for k in ids], ids
+
+
+def dump_sample(n: int):
+    """Sorted indices of the transcripts whose outputs --dump-outputs writes: fixed by DUMP_SEED and n alone."""
+    import numpy as np
+    rng = np.random.default_rng(DUMP_SEED)
+    return np.sort(rng.choice(n, size=min(n, DUMP_TRANSCRIPTS), replace=False))
+
+
+def write_dump(out_dir: str, ids, outputs: dict) -> None:
+    """outputs: transcript index -> (acc, cond) of that transcript."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for k, name in enumerate(("acc", "cond")):
+        arr = np.concatenate([np.asarray(outputs[int(g)][k], np.float32) for g in ids])
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
+    np.save(os.path.join(out_dir, "transcript_index.npy"), np.asarray(ids, np.float64))
+    np.save(os.path.join(out_dir, "lengths.npy"), np.array([len(outputs[int(g)][0]) for g in ids], np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -249,6 +276,19 @@ def ours(args, rank: int, local_rank: int, world: int) -> None:
     t_wall1 = time.perf_counter()
     r.sync()
     c1 = r.counters()
+    if args.dump_outputs:
+        # what the last timed step left on the device, fetched outside the timed region
+        res = r.fetch()
+        pos = {int(g): j for j, g in enumerate(my_ids)}
+        dump_ids = dump_sample(len(all_seqs))
+        mine = {int(g): tuple(np.array(x) for x in res[pos[int(g)]]) for g in dump_ids if int(g) in pos}
+        del res
+        parts = [mine]
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, mine)
+        if rank == 0:
+            write_dump(args.dump_outputs, dump_ids, {g: v for part in parts for g, v in part.items()})
     ms_total = e0.elapsed_time(e1)
     clocks = sampler.stop(t_wall0, t_wall1) if sampler else None
     ms_step = ms_total / args.steps
@@ -262,7 +302,7 @@ def ours(args, rank: int, local_rank: int, world: int) -> None:
     acc_off, cond_off, total = packed_layout(lens)
     out = torch.empty(max(total, 1), dtype=torch.float32).pin_memory().numpy()
     r.run_batch(seqs, out=out)  # warm (page-locked arenas of the library)
-    e2e_steps = 2
+    e2e_steps = args.steps
     c2 = r.counters()
     barrier()
     t0 = time.perf_counter()
@@ -413,7 +453,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--transcripts", type=int, default=N_TRANSCRIPTS,
                     help="take the first N transcripts of the cfg2 stream (default: the whole config, 100,000)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's outputs for a fixed sample of transcripts to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

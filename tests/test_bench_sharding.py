@@ -32,6 +32,23 @@ def test_rank_shards_partition_the_dataset_and_are_balanced():
         assert max(loads) - min(loads) <= int(lens.max()), (world, loads)
 
 
+def test_dump_sample_is_fixed_and_within_64_mb(tmp_path):
+    """--dump-outputs: the same transcripts every run, and at most 64 MB of float32 even if all were 5,000 nt."""
+    bench = _bench()
+    ids = bench.dump_sample(100_000)
+    assert np.array_equal(ids, bench.dump_sample(100_000))
+    assert len(np.unique(ids)) == len(ids) == bench.DUMP_TRANSCRIPTS and ids.min() >= 0 and ids.max() < 100_000
+    assert len(ids) * 2 * 5000 * 4 <= 64 << 20
+    assert np.array_equal(bench.dump_sample(10), np.arange(10))
+    outputs = {int(g): (np.full(int(g) % 7, g, np.float32), np.full(int(g) % 7, -g, np.float32)) for g in ids}
+    bench.write_dump(str(tmp_path), ids, outputs)
+    acc, cond = np.load(tmp_path / "acc.npy"), np.load(tmp_path / "cond.npy")
+    assert acc.dtype == cond.dtype == np.float32
+    assert np.array_equal(acc, np.concatenate([outputs[int(g)][0] for g in ids])) and np.array_equal(cond, -acc)
+    assert np.array_equal(np.load(tmp_path / "transcript_index.npy"), ids.astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "lengths.npy"), (ids % 7).astype(np.float64))
+
+
 def test_split_matches_the_cpp_partitioner_rule():
     """priblast_b200.distributed.lpt_shard = csrc/host/db_format.cpp lpt_partition: longest first onto the least loaded
     part, ties to the lowest part index."""

@@ -3,6 +3,8 @@ to run without CUDA (no fallback), and its host-only record writer reproduces th
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -38,13 +40,18 @@ def test_invalid_arguments_are_status_codes_not_exit():
 
 
 def test_no_cpu_fallback_without_gpu():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
-    from priblast_b200 import Raccess, _capi
-    with pytest.raises(_capi.PribError) as e:
-        Raccess(70, 5)
-    assert e.value.code == -2  # PRIB_ECUDA
+    """In a process that sees no CUDA device (any GPU of the machine hidden), creating a context fails."""
+    code = ("import sys\n"
+            "sys.path.insert(0, sys.argv[1])\n"
+            "from priblast_b200 import Raccess, _capi\n"
+            "try:\n"
+            "    Raccess(70, 5)\n"
+            "except _capi.PribError as e:\n"
+            "    sys.exit(0 if e.code == -2 else 3)\n"  # -2: PRIB_ECUDA
+            "sys.exit(4)\n")
+    p = subprocess.run([sys.executable, "-c", code, ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                       capture_output=True, text=True)
+    assert p.returncode == 0, p.stderr
 
 
 def test_mirror_argument_errors():
