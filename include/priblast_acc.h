@@ -35,11 +35,15 @@ typedef struct prib_ctx prib_ctx;
 /* Constructor arguments of `Raccess(db_name, w, delta, path)` (raccess.hpp:39-58) that matter to the
  * computation, plus device selection. */
 typedef struct prib_acc_params {
-  int32_t maximal_span;          /* W: reference `-w`, default 70 (db_construction_parameters.hpp:48) */
-  int32_t min_accessible_length; /* delta: reference `-d`, default 5; must be > 1 (raccess.hpp:47)   */
+  int32_t maximal_span;          /* W: reference `-w`, default 70 (db_construction_parameters.hpp:48);
+                                    1..1000 (above 200: the wide-span FP64 engine in modes 0 and 1)   */
+  int32_t min_accessible_length; /* delta: reference `-d`, default 5; must be > 1 (raccess.hpp:47);
+                                    2..1000, and may exceed W                                         */
   int32_t device;                /* CUDA device ordinal                                               */
   int32_t mode;                  /* 0 = auto: FP32 span-scaled engine with on-GPU FP64 re-run of
-                                    range-flagged sequences; 1 = FP64 engine only; 2 = exact: the
+                                    range-flagged sequences; 1 = FP64 engine only (modes 0 and 1 at
+                                    W > 200: FP64 span-scaled wide-span engine with on-GPU exact re-run
+                                    of range-flagged sequences); 2 = exact: the
                                     reference's own log-domain arithmetic (float-table logsumexp,
                                     raccess.cpp:414-419, in its summation order) on the GPU: results are
                                     bit-identical to the reference built without FMA contraction     */
@@ -64,6 +68,8 @@ typedef struct prib_acc_counters {
   int64_t fp64_rerun_sequences;  /* sequences the FP32 engine flagged and the FP64 engine recomputed */
   int64_t fp32_flagged[4];       /* sequences whose FIRST FP32 pass left the safe range: [0] inside values too
                                     large, [1] inside too small, [2] outside too large, [3] outside too small */
+  int64_t exact_rerun_sequences; /* sequences the wide-span engine (W > 200) flagged and the exact engine
+                                    recomputed */
 } prib_acc_counters;
 
 /* Replaces the `Raccess` constructor.  One context per GPU; not re-entrant per context. */

@@ -42,6 +42,7 @@ class AccCounters(ctypes.Structure):
         ("phase_ms", ctypes.c_double * 7),
         ("fp64_rerun_sequences", ctypes.c_int64),
         ("fp32_flagged", ctypes.c_int64 * 4),
+        ("exact_rerun_sequences", ctypes.c_int64),
     ]
 
 

@@ -20,10 +20,10 @@ NVCC_FLAGS = [
     "-ccbin", HOST_CXX,
 ]
 
-SOURCES = ["acc_kernels.cu", "acc_exact.cu", "sa_gpu.cu", "acc_tables.cpp"]
+SOURCES = ["acc_kernels.cu", "acc_exact.cu", "acc_wide.cu", "sa_gpu.cu", "acc_tables.cpp"]
 # the exact engine reproduces the reference's IEEE arithmetic bit for bit: no FMA contraction in that TU
 PER_SOURCE_FLAGS = {"acc_exact.cu": ["-fmad=false"]}
-DEPS = SOURCES + ["acc_core.h", "acc_tile.h", "acc_tables.h", "acc_exact.h", "turner_params.h", "turner_blob.c",
+DEPS = SOURCES + ["acc_core.h", "acc_tile.h", "acc_tables.h", "acc_exact.h", "acc_wide.h", "turner_params.h", "turner_blob.c",
                   os.path.join("..", "..", "include", "priblast_acc.h")]
 
 

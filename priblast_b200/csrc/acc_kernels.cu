@@ -9,7 +9,8 @@
 // Every kernel exists for float and double band arithmetic.  The float engine (span-scaled, range
 // guarded) is the fast path (spans up to kFp32MaxSpan); sequences whose stored values leave the safe range
 // are flagged on the device and re-run by the double engine inside the same prib_acc_compute call, on
-// the GPU.  There is no CPU path.
+// the GPU.  Spans above kMaxSpan run the wide-span FP64 engine (acc_wide.cu), whose flagged sequences are
+// re-run by the exact engine (acc_exact.cu) the same way.  There is no CPU path.
 #include <cuda_runtime.h>
 #include <nvtx3/nvToolsExt.h>  // header-only NVTX v3: ranges show up in Nsight Systems / ncu --nvtx, cost nothing otherwise
 
@@ -27,6 +28,7 @@
 #include "acc_exact.h"
 #include "acc_tables.h"
 #include "acc_tile.h"
+#include "acc_wide.h"
 
 using namespace prib;
 
@@ -664,8 +666,9 @@ struct prib_ctx {
   } pipe;
   Engine<float> e32;
   Engine<double> e64;
-  ExactEngine *ex = nullptr;  // mode 2: the reference's own arithmetic (acc_exact.h)
+  ExactEngine *ex = nullptr;  // mode 2, and the re-run of the wide engine: the reference's own arithmetic (acc_exact.h)
   long long ex_max_cols = 0;
+  WideEngine *wide = nullptr;  // spans above kMaxSpan in modes 0 and 1 (acc_wide.h)
   float *d_log = nullptr;
   int grid_tiles = 0;
   char *d_tile_scratch = nullptr;
@@ -1001,12 +1004,7 @@ int run_batch(prib_ctx *c, const Batch &b, bool timed) {
   return PRIB_OK;
 }
 
-// mode 2: every kernel of acc_exact.cu for one batch (phase events in the same slots as the fast engines)
-int run_batch_exact(prib_ctx *c, const Batch &b) {
-  if (settle_phases(c) != PRIB_OK) return PRIB_ECUDA;
-  const long long used = exact_state_bytes_per_column(c->W) * b.NC;
-  if (ensure_state(c, used) != PRIB_OK) return PRIB_ECUDA;
-  if (used > c->cnt.dp_state_bytes_used) c->cnt.dp_state_bytes_used = used;
+ExactBatch exact_batch(prib_ctx *c, const Batch &b) {
   ExactBatch eb;
   eb.NC = b.NC;
   eb.n = b.n;
@@ -1017,9 +1015,35 @@ int run_batch_exact(prib_ctx *c, const Batch &b) {
   eb.acc_off = b.d_acc_off;
   eb.cond_off = b.d_cond_off;
   eb.out = c->d_out;
+  return eb;
+}
+
+// mode 2 and the re-run of the wide engine's flagged sequences: every kernel of acc_exact.cu for one batch (phase
+// events in the same slots as the fast engines)
+int run_batch_exact(prib_ctx *c, const Batch &b, bool timed) {
+  if (timed && settle_phases(c) != PRIB_OK) return PRIB_ECUDA;
+  const long long used = exact_state_bytes_per_column(c->W) * b.NC;
+  if (ensure_state(c, used) != PRIB_OK) return PRIB_ECUDA;
+  if (used > c->cnt.dp_state_bytes_used) c->cnt.dp_state_bytes_used = used;
   int launches = 0;
-  const int e = exact_run(c->ex, eb, c->d_state, c->stream, c->evp, &launches);
+  const int e = exact_run(c->ex, exact_batch(c, b), c->d_state, c->stream, timed ? c->evp : nullptr, &launches);
   if (e != 0) return fail(PRIB_ECUDA, std::string("exact engine: ") + cudaGetErrorString((cudaError_t)e));
+  if (timed) c->phases_pending = true;
+  c->cnt.kernel_launches += launches;
+  c->cnt.batches += 1;
+  return PRIB_OK;
+}
+
+// spans above kMaxSpan (modes 0 and 1): every kernel of acc_wide.cu for one batch; flags come back like the FP32
+// engine's
+int run_batch_wide(prib_ctx *c, const Batch &b) {
+  if (settle_phases(c) != PRIB_OK) return PRIB_ECUDA;
+  const long long used = wide_state_bytes_per_column(c->W) * b.NC;
+  if (ensure_state(c, used) != PRIB_OK) return PRIB_ECUDA;
+  if (used > c->cnt.dp_state_bytes_used) c->cnt.dp_state_bytes_used = used;
+  int launches = 0;
+  const int e = wide_run(c->wide, exact_batch(c, b), b.d_flags, c->d_bad, c->d_state, c->stream, c->evp, &launches);
+  if (e != 0) return fail(PRIB_ECUDA, std::string("wide-span engine: ") + cudaGetErrorString((cudaError_t)e));
   c->phases_pending = true;
   c->cnt.kernel_launches += launches;
   c->cnt.batches += 1;
@@ -1145,7 +1169,7 @@ int compute_prologue(prib_ctx *c) {
   CU(cudaMemsetAsync(c->d_out, 0, (size_t)std::max<long long>(c->out_floats, 1) * sizeof(float), c->stream));
   CU(cudaMemsetAsync(c->d_bad, 0, sizeof(int32_t), c->stream));
   const long long nflags = (long long)c->seq_len.size();
-  if (c->use_fp32 && c->h_flags_cap < nflags) {
+  if ((c->use_fp32 || c->wide) && c->h_flags_cap < nflags) {
     CU(cudaStreamSynchronize(c->stream));
     if (c->h_flags) cudaFreeHost(c->h_flags);
     c->h_flags = nullptr;
@@ -1160,11 +1184,14 @@ int compute_prologue(prib_ctx *c) {
 // All kernels of one staged batch, and the copy of its range flags behind them (no wait).
 int launch_staged_batch(prib_ctx *c, const Batch &b) {
   if (b.n == 0) return PRIB_OK;
-  int rc = c->ex ? run_batch_exact(c, b) : c->use_fp32 ? run_batch<float>(c, b, true) : run_batch<double>(c, b, true);
+  int rc = c->prm.mode == 2 ? run_batch_exact(c, b, true)
+           : c->wide        ? run_batch_wide(c, b)
+           : c->use_fp32    ? run_batch<float>(c, b, true)
+                            : run_batch<double>(c, b, true);
   if (rc != PRIB_OK) return rc;
   c->cnt.sequences += b.n;
   c->cnt.nucleotides += b.nt;
-  if (c->use_fp32) {
+  if (c->use_fp32 || c->wide) {
     CU(cudaMemcpyAsync(c->h_flags + c->pipe.fpos, b.d_flags, sizeof(int32_t) * (size_t)b.n, cudaMemcpyDeviceToHost, c->stream));
     c->pipe.fpos += b.n;
   }
@@ -1187,10 +1214,10 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   *out = nullptr;
   if (params->min_accessible_length <= 1)
     return fail(PRIB_EINVAL, "Error: -d option must be greater than 1");  // raccess.hpp:47-50
-  if (params->maximal_span < 1 || params->maximal_span > kMaxSpan)
-    return fail(PRIB_EINVAL, "maximal span must be in 1.." + std::to_string((int)kMaxSpan));
-  if (params->min_accessible_length > kMaxLoop)
-    return fail(PRIB_EINVAL, "minimum accessible length above 30 is not supported");
+  if (params->maximal_span < 1 || params->maximal_span > kWideSpan)
+    return fail(PRIB_EINVAL, "maximal span must be in 1.." + std::to_string((int)kWideSpan));
+  if (params->min_accessible_length > kWideSpan)
+    return fail(PRIB_EINVAL, "minimum accessible length must be in 2.." + std::to_string((int)kWideSpan));
   if (params->mode < 0 || params->mode > 2)
     return fail(PRIB_EINVAL, "mode must be 0 (auto), 1 (fp64 only) or 2 (exact: reference arithmetic)");
   int ndev = 0;
@@ -1207,7 +1234,8 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   const char *pe = getenv("PRIB_PRECISION");
   int fp32_max_span = kFp32MaxSpan;
   if (const char *me = getenv("PRIB_FP32_MAXSPAN")) fp32_max_span = atoi(me);  // tuning knob
-  c->use_fp32 = params->mode == 0 && c->W <= fp32_max_span && !(pe && strcmp(pe, "fp64") == 0);
+  c->use_fp32 = params->mode == 0 && c->W <= fp32_max_span && c->W <= kMaxSpan && !(pe && strcmp(pe, "fp64") == 0);
+  const bool wide = c->W > kMaxSpan && params->mode != 2;  // the tile kernels stop at kMaxSpan
   auto bail = [&](int code) {
     std::string keep = g_err;
     prib_acc_destroy(c);
@@ -1234,8 +1262,17 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   CUB(cudaGetDeviceProperties(&prop, params->device));
   c->grid_tiles = prop.multiProcessorCount;
   std::string err;
-  int rc = setup_engine<double>(c, ScaleSpec(), prop.sharedMemPerBlockOptin, err);
-  if (rc != PRIB_OK) return bail(rc == PRIB_EINVAL ? fail(rc, err) : rc);
+  int rc = PRIB_OK;
+  if (c->W <= kMaxSpan) {
+    rc = setup_engine<double>(c, ScaleSpec(), prop.sharedMemPerBlockOptin, err);
+    if (rc != PRIB_OK) return bail(rc == PRIB_EINVAL ? fail(rc, err) : rc);
+  }
+  if (wide) {
+    double klog2 = default_scale_wide().klog2;
+    if (const char *e = getenv("PRIB_WIDE_KLOG2")) klog2 = atof(e);  // tuning knob (profiles/scale_scan.py <W> <n> wide)
+    c->wide = wide_create(c->W, c->delta, klog2, err);
+    if (!c->wide) return bail(fail(PRIB_ECUDA, err));
+  }
   if (c->use_fp32) {
     ScaleSpec sp32 = default_scale_fp32();
     if (const char *e = getenv("PRIB_KLOG2")) sp32.klog2 = atof(e);  // tuning knobs (profiles/scale_scan.py)
@@ -1244,13 +1281,13 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
     rc = setup_engine<float>(c, sp32, prop.sharedMemPerBlockOptin, err);
     if (rc != PRIB_OK) return bail(rc == PRIB_EINVAL ? fail(rc, err) : rc);
   }
-  if (params->mode == 2) {
+  if (params->mode == 2 || wide) {
     c->ex = exact_create(c->W, c->delta, err);
     if (!c->ex) return bail(fail(PRIB_ECUDA, err));
   }
   const size_t scr64 = (size_t)2 * (c->W + 4) * c->e64.TC * sizeof(double);
   const size_t scr32 = (size_t)2 * (c->W + 4) * c->e32.TC * sizeof(float);
-  CUB(cudaMalloc(&c->d_tile_scratch, (size_t)c->grid_tiles * std::max(scr64, scr32)));
+  if (!wide) CUB(cudaMalloc(&c->d_tile_scratch, (size_t)c->grid_tiles * std::max(scr64, scr32)));
 
   size_t free_b = 0, total_b = 0;
   CUB(cudaMemGetInfo(&free_b, &total_b));
@@ -1283,6 +1320,7 @@ void prib_acc_destroy(prib_ctx *c) {
   c->e32.release();
   c->e64.release();
   exact_destroy(c->ex);
+  wide_destroy(c->wide);
   cudaFree(c->d_log);
   if (c->h_stage) cudaFreeHost(c->h_stage);
   if (c->h_arena) cudaFreeHost(c->h_arena);
@@ -1317,7 +1355,7 @@ int prib_acc_stage(prib_ctx *c, int32_t n, const char *const *seq, const int32_t
     for (int k = 0; k < n; k++) total_len += len[k] > 0 ? len[k] : 0;
     c->set_budget(n > 0 && total_len / n > 8192 ? c->budget_long : c->budget_default);
   }
-  const long long max_cols = c->ex ? c->ex_max_cols : c->use_fp32 ? c->e32.max_cols : c->e64.max_cols;
+  const long long max_cols = c->prm.mode == 2 ? c->ex_max_cols : c->use_fp32 ? c->e32.max_cols : c->e64.max_cols;
   for (int k = 0; k < n; k++) {
     if (len[k] < 0) return fail(PRIB_EINVAL, "negative sequence length");
     if (layout_columns(len[k]) + 2 * kPad > std::min(max_cols, c->e64.max_cols))
@@ -1399,7 +1437,7 @@ int prib_acc_compute(prib_ctx *c) {
   // range flags of all batches come back with ONE wait after the last batch (each batch has its own flag array)
   long long fpos = 0;
   std::vector<int> flagged;
-  if (c->use_fp32) {
+  if (c->use_fp32 || c->wide) {
     CU(cudaStreamSynchronize(c->stream));
     fpos = 0;
     for (size_t bi = 0; bi < c->n_batches; ++bi) {
@@ -1407,14 +1445,15 @@ int prib_acc_compute(prib_ctx *c) {
       for (int k = 0; k < b.n; k++)
         if (const int bits = c->h_flags[fpos + k]) {
           flagged.push_back(b.ids[k]);
-          for (int q = 0; q < 4; q++)
+          for (int q = 0; q < 4 && c->use_fp32; q++)
             if (bits & (1 << q)) c->cnt.fp32_flagged[q] += 1;
         }
       fpos += b.n;
     }
   }
   if (!flagged.empty()) {
-    // re-run in double, on the GPU, writing to the same places of the output image
+    // re-run in double (FP32 engine) or in the exact engine (wide engine), on the GPU, writing to the same places of
+    // the output image
     const size_t nall = c->seq_len.size();
     std::vector<long long> acc_abs(nall), cond_abs(nall);
     long long o = 0;
@@ -1440,15 +1479,15 @@ int prib_acc_compute(prib_ctx *c) {
     const size_t meta_keep = c->h_meta_used;
     std::vector<Batch> fb;
     size_t nfb = 0;
-    rc = partition(c, flagged, c->e64.max_cols, acc_abs, cond_abs, fb, &nfb, rerun_begin);
+    rc = partition(c, flagged, c->wide ? c->ex_max_cols : c->e64.max_cols, acc_abs, cond_abs, fb, &nfb, rerun_begin);
     for (Batch &b : fb) {
-      if (rc == PRIB_OK) rc = run_batch<double>(c, b, false);
-      if (rc == PRIB_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) rc = fail(PRIB_ECUDA, "fp64 re-run failed");
+      if (rc == PRIB_OK) rc = c->wide ? run_batch_exact(c, b, false) : run_batch<double>(c, b, false);
+      if (rc == PRIB_OK && cudaStreamSynchronize(c->stream) != cudaSuccess) rc = fail(PRIB_ECUDA, "re-run failed");
       free_batch(b);
     }
     c->h_meta_used = meta_keep;  // (compute may be called again on the same staged batches)
     if (rc != PRIB_OK) return rc;
-    c->cnt.fp64_rerun_sequences += (long long)flagged.size();
+    (c->wide ? c->cnt.exact_rerun_sequences : c->cnt.fp64_rerun_sequences) += (long long)flagged.size();
   }
   CU(cudaEventRecord(c->evk1, c->stream));
   c->kernel_timed = false;

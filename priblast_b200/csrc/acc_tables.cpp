@@ -2,23 +2,24 @@
 
 #include <cmath>
 #include <cstring>
+#include <limits>
 
 #include "turner_params.h"
 
 namespace prib {
 
-template <typename real>
-bool build_tables(int W, int delta, const ScaleSpec &spec, HostTablesT<real> &out, std::string &err) {
+template <typename real, int CAP>
+bool build_tables(int W, int delta, const ScaleSpec &spec, HostTablesT<real, CAP> &out, std::string &err) {
   const prib_turner_params *p = prib_turner_embedded();
   if (!p) {
     err = "embedded Turner parameter blob missing or corrupt";
     return false;
   }
-  if (W < 1 || W > kMaxSpan) {
-    err = "maximal span out of range (1.." + std::to_string((int)kMaxSpan) + ")";
+  if (W < 1 || W > CAP) {
+    err = "maximal span out of range (1.." + std::to_string((int)CAP) + ")";
     return false;
   }
-  typename Core<real>::SmallTables &T = out.small;
+  typename Core<real, CAP>::SmallTables &T = out.small;
   std::memset(&T, 0, sizeof(T));
   // energy_par.hpp:12-13; every scaled value is (-E*10)/kT as in raccess.hpp:105-158
   const double kT = (p->temperature_c + p->k0) * p->gasconst;
@@ -33,6 +34,14 @@ bool build_tables(int W, int delta, const ScaleSpec &spec, HostTablesT<real> &ou
   T.kacc = kap * kap / (cA * cB);
   T.kmul[0] = kpow(delta) / (cA * cB);
   T.kmul[1] = kpow(delta + 1) / (cA * cB);
+  // kmul is stored as `real`.  CalcMultiProbability has terms only for windows w <= W - 4 (a multiloop needs a
+  // span-5 branch beside the window), so kmul only has to be a normal number up to delta + 1 <= W - 4; for a wider
+  // window both sums are empty and an underflowed kmul multiplies 0.  (FP32: kappa^197 / (cA cB) = 2^-109 at
+  // W = 200 with the default scale.)
+  if (delta + 1 <= W - 4 && !(T.kmul[1] >= std::numeric_limits<real>::min())) {
+    err = "span scale too strong for the minimum accessible length (kappa^(delta+1) / (cA cB) underflows)";
+    return false;
+  }
   T.e_mlbase = kap * std::exp(MLbase);
   T.e_mlintern = std::exp(MLintern);
   T.e_mlclose = std::exp(MLclosing + MLintern);
@@ -49,12 +58,12 @@ bool build_tables(int W, int delta, const ScaleSpec &spec, HostTablesT<real> &ou
     ninio[i] = sc(v);
   }
   // HairpinEnergy length term incl. the logarithmic extrapolation (raccess.cpp:823)
-  for (int d = 0; d < kMaxSpan + 8; d++) {
+  for (int d = 0; d < CAP + 8; d++) {
     double q = d <= 30 ? hairpin[d] : hairpin[30] - p->lxc37 * std::log(d / 30.) * 10. / kT;
     T.e_hairpin[d] = cA * kpow(d) * std::exp(q);
     T.sB[d] = cB * kpow(-d);
     T.us[d] = kpow(-d) / cA;
-    if (d + 1 < kMaxSpan + 8) T.hpB[d + 1] = kpow(d + 2) / cB * std::exp(q);  // indexed by dd = loop size + 1
+    if (d + 1 < CAP + 8) T.hpB[d + 1] = kpow(d + 2) / cB * std::exp(q);  // indexed by dd = loop size + 1
   }
   for (int u = 0; u < 32; u++) T.e_bulge[u] = u <= 30 ? kpow(u) * std::exp(bulge[u]) : 0.0;
   for (int k = 0; k < 8; k++) T.cg[k] = std::exp(ninio[k < 6 ? k : 6]);
@@ -115,8 +124,10 @@ bool build_tables(int W, int delta, const ScaleSpec &spec, HostTablesT<real> &ou
   return true;
 }
 
-template bool build_tables<double>(int, int, const ScaleSpec &, HostTablesT<double> &, std::string &);
-template bool build_tables<float>(int, int, const ScaleSpec &, HostTablesT<float> &, std::string &);
+template bool build_tables<double, kMaxSpan>(int, int, const ScaleSpec &, HostTablesT<double> &, std::string &);
+template bool build_tables<float, kMaxSpan>(int, int, const ScaleSpec &, HostTablesT<float> &, std::string &);
+template bool build_tables<double, kWideSpan>(int, int, const ScaleSpec &, HostTablesT<double, kWideSpan> &,
+                                              std::string &);
 
 void build_layout(int n, const char *const *seqs, const int32_t *lens, BatchLayout &out) {
   out.seq_off.resize(n);

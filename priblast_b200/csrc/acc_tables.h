@@ -9,9 +9,9 @@
 
 namespace prib {
 
-template <typename real>
+template <typename real, int CAP = kMaxSpan>
 struct HostTablesT {
-  typename Core<real>::SmallTables small;
+  typename Core<real, CAP>::SmallTables small;
   std::vector<real> e_int11, e_int21, e_int22;
   std::vector<float> log_tbl;  // 2048 x (app, rev)
 };
@@ -37,8 +37,18 @@ inline ScaleSpec default_scale_fp32() {
   return s;
 }
 
-template <typename real>
-bool build_tables(int W, int delta, const ScaleSpec &sc, HostTablesT<real> &out, std::string &err);
+// Span scaling of the wide-span FP64 engine (acc_wide.cu).  Its stored values are range-checked against 2^+-480,
+// so kappa only has to keep Alpha and Beta / Z of the widest cells inside that window: kappa = 2^-klog2 per nt
+// (profiles/scale_scan.py <W> <n> wide, DESIGN.md §2.9); cA = cB = 1.
+inline ScaleSpec default_scale_wide() {
+  ScaleSpec s;
+  s.klog2 = 0.45;
+  return s;
+}
+
+// Instantiated for <float, kMaxSpan>, <double, kMaxSpan> and <double, kWideSpan>.
+template <typename real, int CAP>
+bool build_tables(int W, int delta, const ScaleSpec &sc, HostTablesT<real, CAP> &out, std::string &err);
 
 // Column layout of one batch (DESIGN.md §3): sequence k occupies columns seq_off[k] .. seq_off[k]+len[k]
 // (left indices 0..L), followed by >= kPad zero columns; the first sequence starts at kPad.

@@ -84,6 +84,9 @@ static void usage() {
       "                        [-w MaximalSpan] [-d MinAccessibleLength] [-c ChunkSize] [-a block|heap|dynamic]\n"
       "                        [-p TmpPath] [-m auto|fp64|exact]\n"
       "defaults: -r 0 -s 8 -w 70 -d 5 -a heap -c INT_MAX   (reference: main.cpp:43-73)\n"
+      "ranges: -w 1..1000, -d 2..1000 (-d may exceed -w); above -w 200, auto and fp64 run the FP64 wide-span engine\n"
+      "   (.acc within 1e-4 kcal/mol of the reference; sequences whose values leave its range are recomputed by the\n"
+      "   exact engine)\n"
       "-m (extension; also PRIB_ACC_MODE): auto = FP32 span-scaled engine with FP64 re-run (default; .acc within\n"
       "   1e-4 kcal/mol of the reference), fp64, exact = the reference's own arithmetic on the GPU (.acc, hence\n"
       "   the whole database and the ris output, byte-identical to a reference built WITHOUT FMA contraction,\n"
