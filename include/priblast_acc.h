@@ -72,8 +72,23 @@ typedef struct prib_acc_counters {
                                     recomputed */
 } prib_acc_counters;
 
-/* Replaces the `Raccess` constructor.  One context per GPU; not re-entrant per context. */
+/* Replaces the `Raccess` constructor.  One context per GPU; not re-entrant per context.
+ * Same as prib_acc_create_lengths(out, params, 1, &params->min_accessible_length). */
 int prib_acc_create(prib_ctx **out, const prib_acc_params *params);
+
+#define PRIB_MAX_LENGTHS 32
+
+/* A context that computes accessibility for n_lengths minimum accessible lengths in each call: the inside pass, the
+ * outer scans and the outside pass run once per batch, the strand weights and the finalize once per length.  Every
+ * output float equals that of a context created with prib_acc_create for that length alone.
+ *   lengths        : 1 <= n_lengths <= PRIB_MAX_LENGTHS entries, strictly increasing, each checked like
+ *                    min_accessible_length (which is not read); a bad entry is PRIB_EINVAL, named in the message.
+ *   acc_off/cond_off of prib_acc_run and prib_acc_fetch then have n_lengths * n entries: [l * n + k] is sequence k at
+ *                    lengths[l].  With the packed layout of each length back to back, fetch copies the device image
+ *                    straight into a page-locked `out`.
+ * Counters: sequences, nucleotides and the re-run counts count each sequence once (a flagged sequence is re-run once
+ * for all lengths); the last three phase_ms entries sum over the lengths. */
+int prib_acc_create_lengths(prib_ctx **out, const prib_acc_params *params, int32_t n_lengths, const int32_t *lengths);
 void prib_acc_destroy(prib_ctx *ctx);
 
 /* Replaces the loop of `Raccess::Run(seq, acc, cond)` calls (raccess.cpp:42-50) over n sequences.

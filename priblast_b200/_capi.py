@@ -49,6 +49,8 @@ class AccCounters(ctypes.Structure):
 # name -> (restype, argtypes); must list exactly the functions of include/priblast_acc.h
 SIGNATURES = {
     "prib_acc_create": (ctypes.c_int, [ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(AccParams)]),
+    "prib_acc_create_lengths": (ctypes.c_int, [ctypes.POINTER(ctypes.c_void_p), ctypes.POINTER(AccParams),
+                                               ctypes.c_int32, c_i32p]),
     "prib_acc_destroy": (None, [ctypes.c_void_p]),
     "prib_acc_run": (ctypes.c_int, [ctypes.c_void_p, ctypes.c_int32, ctypes.POINTER(ctypes.c_char_p), c_i32p,
                                     ctypes.c_void_p, c_i64p, c_i64p]),
@@ -97,6 +99,8 @@ def load() -> ctypes.CDLL:
     _lib = lib
     return lib
 
+
+MAX_LENGTHS = 32  # PRIB_MAX_LENGTHS
 
 PHASE_NAMES = ["memset", "inside", "outer_scans", "outside", "biloop_left", "biloop_right", "hairpin_finalize"]
 

@@ -755,14 +755,15 @@ __global__ void __launch_bounds__(128) k_ex_finalize(ExCtx c) {
 }  // namespace
 
 struct ExactEngine {
-  int W = 0, delta = 0;
+  int W = 0;
+  std::vector<int> lengths;
   ExTab *d_tab = nullptr;
   double *d_int21 = nullptr, *d_int22 = nullptr;
 };
 
 long long exact_state_bytes_per_column(int W) { return ((long long)kExArr * (W + 2) + kExVec) * 8; }
 
-ExactEngine *exact_create(int W, int delta, std::string &err) {
+ExactEngine *exact_create(int W, const std::vector<int> &lengths, std::string &err) {
   const prib_turner_params *p = prib_turner_embedded();
   if (!p) {
     err = "embedded Turner parameter blob missing or corrupt";
@@ -856,7 +857,7 @@ ExactEngine *exact_create(int W, int delta, std::string &err) {
     ok = cudaFuncSetAttribute(k_ex_outer, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ex_outer_smem(W)) == cudaSuccess;
   if (ok) {
     eng->W = W;
-    eng->delta = delta;
+    eng->lengths = lengths;
     ok = cudaMalloc(&eng->d_tab, sizeof(ExTab)) == cudaSuccess &&
          cudaMalloc(&eng->d_int21, i21.size() * 8) == cudaSuccess &&
          cudaMalloc(&eng->d_int22, i22.size() * 8) == cudaSuccess &&
@@ -885,7 +886,7 @@ int exact_run(ExactEngine *e, const ExactBatch &b, char *d_state, cudaStream_t s
   ExCtx c;
   c.NC = b.NC;
   c.W = e->W;
-  c.delta = e->delta;
+  c.delta = e->lengths[0];
   c.nseq = b.n;
   c.S = b.S;
   c.col_seq = b.col_seq;
@@ -916,14 +917,23 @@ int exact_run(ExactEngine *e, const ExactBatch &b, char *d_state, cudaStream_t s
   EX_EV(3);
   for (int d = W + 1; d >= kTurn; d--, ++nl) k_ex_outside<<<grid, 128, 0, st>>>(c, d);
   EX_EV(4);
-  k_ex_biloop<<<(unsigned)((b.NC + kBiB - 1) / kBiB), kBiB, 0, st>>>(c);
-  ++nl;
-  EX_EV(5);
-  EX_EV(6);
-  k_ex_hairpin<<<grid, 128, 0, st>>>(c);
-  k_ex_finalize<<<grid, 128, 0, st>>>(c);
-  nl += 2;
-  EX_EV(7);
+  for (size_t l = 0; l < e->lengths.size(); ++l) {
+    c.delta = e->lengths[l];
+    c.out = b.out + (long long)l * b.out_stride;
+    // k_ex_hairpin writes only the positions that have a hairpin term: clear the previous length's
+    if (l > 0) {
+      const cudaError_t r = cudaMemsetAsync(c.vec + 2 * c.NC, 0, (size_t)(2 * c.NC) * sizeof(double), st);
+      if (r != cudaSuccess) return (int)r;
+    }
+    k_ex_biloop<<<(unsigned)((b.NC + kBiB - 1) / kBiB), kBiB, 0, st>>>(c);
+    ++nl;
+    EX_EV(5 + 3 * l);
+    EX_EV(6 + 3 * l);
+    k_ex_hairpin<<<grid, 128, 0, st>>>(c);
+    k_ex_finalize<<<grid, 128, 0, st>>>(c);
+    nl += 2;
+    EX_EV(7 + 3 * l);
+  }
 #undef EX_EV
   if (launches) *launches = nl;
   return (int)cudaGetLastError();

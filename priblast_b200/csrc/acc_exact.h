@@ -16,6 +16,7 @@
 #include <stdint.h>
 
 #include <string>
+#include <vector>
 
 namespace prib {
 
@@ -27,17 +28,21 @@ struct ExactBatch {
   const int32_t *seq_len;
   const long long *seq_off;
   const long long *acc_off, *cond_off;  // float offsets into out
-  float *out;
+  float *out;              // output image of the first minimum accessible length
+  long long out_stride;    // floats from the output image of one length to that of the next
 };
 
 struct ExactEngine;  // opaque: device tables
 
 long long exact_state_bytes_per_column(int W);
 // Builds the scaled energy tables (raccess.hpp:105-158) and the two fmath tables from the host libm, exactly
-// as the reference does at static-init time, and uploads them.  Returns nullptr and sets err on failure.
-ExactEngine *exact_create(int W, int delta, std::string &err);
+// as the reference does at static-init time, and uploads them.  lengths: the minimum accessible lengths, increasing.
+// Returns nullptr and sets err on failure.
+ExactEngine *exact_create(int W, const std::vector<int> &lengths, std::string &err);
 void exact_destroy(ExactEngine *e);
-// All kernels of one batch on `stream`; d_state must hold exact_state_bytes_per_column(W) * NC bytes.
+// All kernels of one batch on `stream`; d_state must hold exact_state_bytes_per_column(W) * NC bytes.  The inside,
+// outer and outside passes run once; the hairpin, loop and finalize kernels once per length.  phase_events: 8 events
+// for one length, 3 more per further length (the last three phases of each length).
 // Returns a cudaError_t (0 = ok); *launches receives the number of kernel launches.
 int exact_run(ExactEngine *e, const ExactBatch &b, char *d_state, cudaStream_t stream, cudaEvent_t *phase_events,
               int *launches);

@@ -628,7 +628,7 @@ struct Batch {
 template <typename real>
 struct Engine {
   typedef typename Core<real>::SmallTables ST;
-  ST *d_small = nullptr;
+  std::vector<ST *> d_small;  // one per minimum accessible length (they differ in kmul only)
   real *d_int11 = nullptr, *d_int21 = nullptr, *d_int22 = nullptr;
   int TC = 0;
   size_t tile_smem = 0;
@@ -638,11 +638,11 @@ struct Engine {
   long long max_cols = 0;
 
   void release() {
-    cudaFree(d_small);
+    for (ST *t : d_small) cudaFree(t);
     cudaFree(d_int11);
     cudaFree(d_int21);
     cudaFree(d_int22);
-    d_small = nullptr;
+    d_small.clear();
     d_int11 = d_int21 = d_int22 = nullptr;
   }
 };
@@ -651,11 +651,16 @@ struct Engine {
 
 struct prib_ctx {
   prib_acc_params prm{};
-  int W = 70, delta = 5;
+  int W = 70;
+  // Minimum accessible lengths, increasing.  The inside and outside passes, the outer scans and the range flags do not
+  // depend on delta, so they run once per batch; the strand weights and the finalize run once per length.
+  std::vector<int> lengths;
   bool use_fp32 = true;
   cudaStream_t own_stream = nullptr, stream = nullptr;
   cudaEvent_t ev0 = nullptr, ev1 = nullptr, evk0 = nullptr, evk1 = nullptr;
-  cudaEvent_t evp[PRIB_NUM_PHASES + 1] = {};
+  // phase events: evp[0..4] open the first five phases; length l closes biloop_left, biloop_right and
+  // hairpin_finalize with evp[5 + 3 l], evp[6 + 3 l] and evp[7 + 3 l] (PRIB_NUM_PHASES + 1 events for one length)
+  std::vector<cudaEvent_t> evp;
   bool phases_pending = false, kernel_timed = true, stage_timed = true;
   // prib_acc_run: the stage fills the arena batch by batch and launches each batch as soon as it is staged, so the
   // host copy of batch k + 1 runs under the kernels of batch k (prib_acc_stage / _compute on their own do not)
@@ -694,8 +699,9 @@ struct prib_ctx {
   unsigned char *h_meta = nullptr;  // page-locked per-batch offset arrays (bump-allocated per stage)
   size_t h_meta_cap = 0, h_meta_used = 0;
   size_t n_batches = 0;           // batches[0..n_batches) are live; the rest keep their buffers for reuse
-  float *d_out = nullptr;
-  long long out_floats = 0, out_cap = 0;
+  float *d_out = nullptr;  // length-major: the packed image of length l starts at l * out_floats
+  long long out_floats = 0, out_cap = 0;  // out_floats: one length's image; out_cap: the whole allocation
+  long long image_floats() const { return out_floats * (long long)lengths.size(); }
   bool staged = false, computed = false;
   float *h_stage = nullptr;
   long long h_stage_floats = 0;
@@ -749,14 +755,14 @@ typename Core<real>::Ctx make_ctx(prib_ctx *c, const Batch &b) {
   std::memset(&k, 0, sizeof(k));
   k.NC = b.NC;
   k.W = c->W;
-  k.delta = c->delta;
+  k.delta = c->lengths[0];  // the inside pass stores A_STEM when 2 is one of the lengths
   k.rows = c->W + 4;
   k.nseq = b.n;
   k.S = b.d_S;
   k.col_seq = b.d_col_seq;
   k.seq_len = b.d_seq_len;
   k.seq_off = b.d_seq_off;
-  k.T = e.d_small;
+  k.T = e.d_small[0];
   k.e_int11 = e.d_int11;
   k.e_int21 = e.d_int21;
   k.e_int22 = e.d_int22;
@@ -779,11 +785,11 @@ typename Core<real>::Ctx make_ctx(prib_ctx *c, const Batch &b) {
 
 int settle_phases(prib_ctx *c) {
   if (!c->phases_pending) return PRIB_OK;
-  CU(cudaEventSynchronize(c->evp[PRIB_NUM_PHASES]));
-  for (int p = 0; p < PRIB_NUM_PHASES; p++) {
+  CU(cudaEventSynchronize(c->evp.back()));
+  for (size_t e = 0; e + 1 < c->evp.size(); e++) {  // the last three phases come once per length
     float ms = 0;
-    CU(cudaEventElapsedTime(&ms, c->evp[p], c->evp[p + 1]));
-    c->cnt.phase_ms[p] += ms;
+    CU(cudaEventElapsedTime(&ms, c->evp[e], c->evp[e + 1]));
+    c->cnt.phase_ms[e < 4 ? e : 4 + (e - 4) % 3] += ms;
   }
   c->phases_pending = false;
   return PRIB_OK;
@@ -986,20 +992,27 @@ int run_batch(prib_ctx *c, const Batch &b, bool timed) {
   k_outside_tile<real><<<tgrid, e.TC, e.tile_smem, st>>>(k, TX, ntiles, scratch);
   if (timed) CU(cudaEventRecord(c->evp[4], st));
   nvtxRangePop();
-  nvtxRangePushA("prib:strand_weights");
+  // per length: its delta, its tables and its slice of the output image; the strand-weight arrays are overwritten
   const unsigned bgrid = (unsigned)((b.NC + e.TXb - 1) / e.TXb);
-  launch_biloop<real, true>(k, bgrid, e.TXb, e.bi_smem, st);
-  if (timed) CU(cudaEventRecord(c->evp[5], st));
-  launch_biloop<real, false>(k, bgrid, e.TXb, e.bi_smem, st);
-  if (timed) CU(cudaEventRecord(c->evp[6], st));
-  nvtxRangePop();
-  nvtxRangePushA("prib:finalize");  // the hairpin suffix sums come out of the left strand-weight kernel
-  k_finalize<real><<<grid, kThreads, 0, st>>>(k);
-  if (timed) CU(cudaEventRecord(c->evp[7], st));
-  nvtxRangePop();
+  for (size_t l = 0; l < c->lengths.size(); ++l) {
+    typename Core<real>::Ctx kl = k;
+    kl.delta = c->lengths[l];
+    kl.T = e.d_small[l];
+    kl.out = c->d_out + (long long)l * c->out_floats;
+    nvtxRangePushA("prib:strand_weights");
+    launch_biloop<real, true>(kl, bgrid, e.TXb, e.bi_smem, st);
+    if (timed) CU(cudaEventRecord(c->evp[5 + 3 * l], st));
+    launch_biloop<real, false>(kl, bgrid, e.TXb, e.bi_smem, st);
+    if (timed) CU(cudaEventRecord(c->evp[6 + 3 * l], st));
+    nvtxRangePop();
+    nvtxRangePushA("prib:finalize");  // the hairpin suffix sums come out of the left strand-weight kernel
+    k_finalize<real><<<grid, kThreads, 0, st>>>(kl);
+    if (timed) CU(cudaEventRecord(c->evp[7 + 3 * l], st));
+    nvtxRangePop();
+  }
   CU(cudaGetLastError());
   if (timed) c->phases_pending = true;
-  c->cnt.kernel_launches += 6;
+  c->cnt.kernel_launches += 3 + 3 * (long long)c->lengths.size();
   c->cnt.batches += 1;
   return PRIB_OK;
 }
@@ -1015,6 +1028,7 @@ ExactBatch exact_batch(prib_ctx *c, const Batch &b) {
   eb.acc_off = b.d_acc_off;
   eb.cond_off = b.d_cond_off;
   eb.out = c->d_out;
+  eb.out_stride = c->out_floats;
   return eb;
 }
 
@@ -1026,7 +1040,7 @@ int run_batch_exact(prib_ctx *c, const Batch &b, bool timed) {
   if (ensure_state(c, used) != PRIB_OK) return PRIB_ECUDA;
   if (used > c->cnt.dp_state_bytes_used) c->cnt.dp_state_bytes_used = used;
   int launches = 0;
-  const int e = exact_run(c->ex, exact_batch(c, b), c->d_state, c->stream, timed ? c->evp : nullptr, &launches);
+  const int e = exact_run(c->ex, exact_batch(c, b), c->d_state, c->stream, timed ? c->evp.data() : nullptr, &launches);
   if (e != 0) return fail(PRIB_ECUDA, std::string("exact engine: ") + cudaGetErrorString((cudaError_t)e));
   if (timed) c->phases_pending = true;
   c->cnt.kernel_launches += launches;
@@ -1042,7 +1056,7 @@ int run_batch_wide(prib_ctx *c, const Batch &b) {
   if (ensure_state(c, used) != PRIB_OK) return PRIB_ECUDA;
   if (used > c->cnt.dp_state_bytes_used) c->cnt.dp_state_bytes_used = used;
   int launches = 0;
-  const int e = wide_run(c->wide, exact_batch(c, b), b.d_flags, c->d_bad, c->d_state, c->stream, c->evp, &launches);
+  const int e = wide_run(c->wide, exact_batch(c, b), b.d_flags, c->d_bad, c->d_state, c->stream, c->evp.data(), &launches);
   if (e != 0) return fail(PRIB_ECUDA, std::string("wide-span engine: ") + cudaGetErrorString((cudaError_t)e));
   c->phases_pending = true;
   c->cnt.kernel_launches += launches;
@@ -1054,10 +1068,13 @@ template <typename real>
 int setup_engine(prib_ctx *c, const ScaleSpec &spec, size_t smem_max, std::string &err) {
   Engine<real> &e = engine<real>(c);
   HostTablesT<real> tab;
-  if (!build_tables(c->W, c->delta, spec, tab, err)) return PRIB_EINVAL;
   typedef typename Core<real>::SmallTables ST;
-  CU(cudaMalloc(&e.d_small, sizeof(ST)));
-  CU(cudaMemcpy(e.d_small, &tab.small, sizeof(ST), cudaMemcpyHostToDevice));
+  for (int delta : c->lengths) {  // the small tables per length; everything uploaded below depends on no delta
+    if (!build_tables(c->W, delta, spec, tab, err)) return PRIB_EINVAL;
+    e.d_small.push_back(nullptr);
+    CU(cudaMalloc(&e.d_small.back(), sizeof(ST)));
+    CU(cudaMemcpy(e.d_small.back(), &tab.small, sizeof(ST), cudaMemcpyHostToDevice));
+  }
   CU(cudaMalloc(&e.d_int11, tab.e_int11.size() * sizeof(real)));
   CU(cudaMemcpy(e.d_int11, tab.e_int11.data(), tab.e_int11.size() * sizeof(real), cudaMemcpyHostToDevice));
   CU(cudaMalloc(&e.d_int21, tab.e_int21.size() * sizeof(real)));
@@ -1166,7 +1183,7 @@ int settle_kernel_time(prib_ctx *c) {
 int compute_prologue(prib_ctx *c) {
   if (settle_kernel_time(c) != PRIB_OK) return PRIB_ECUDA;
   CU(cudaEventRecord(c->evk0, c->stream));
-  CU(cudaMemsetAsync(c->d_out, 0, (size_t)std::max<long long>(c->out_floats, 1) * sizeof(float), c->stream));
+  CU(cudaMemsetAsync(c->d_out, 0, (size_t)std::max<long long>(c->image_floats(), 1) * sizeof(float), c->stream));
   CU(cudaMemsetAsync(c->d_bad, 0, sizeof(int32_t), c->stream));
   const long long nflags = (long long)c->seq_len.size();
   if ((c->use_fp32 || c->wide) && c->h_flags_cap < nflags) {
@@ -1211,13 +1228,27 @@ const char *prib_version(void) { return "priblast-b200 0.2 (sm_100a; fp32 span-s
 
 int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   if (!out || !params) return fail(PRIB_EINVAL, "null argument");
+  return prib_acc_create_lengths(out, params, 1, &params->min_accessible_length);
+}
+
+int prib_acc_create_lengths(prib_ctx **out, const prib_acc_params *params, int32_t n_lengths, const int32_t *lengths) {
+  if (!out || !params || !lengths) return fail(PRIB_EINVAL, "null argument");
   *out = nullptr;
-  if (params->min_accessible_length <= 1)
-    return fail(PRIB_EINVAL, "Error: -d option must be greater than 1");  // raccess.hpp:47-50
+  if (n_lengths < 1 || n_lengths > PRIB_MAX_LENGTHS)
+    return fail(PRIB_EINVAL, "number of minimum accessible lengths must be in 1.." + std::to_string(PRIB_MAX_LENGTHS));
+  // a list names the offending entry; a single length keeps the messages of the reference's one -d value
+  auto bad_length = [&](int l, const std::string &msg) {
+    return fail(PRIB_EINVAL, n_lengths == 1 ? msg : "lengths[" + std::to_string(l) + "] = " + std::to_string(lengths[l]) + ": " + msg);
+  };
+  for (int l = 0; l < n_lengths; l++)
+    if (lengths[l] <= 1) return bad_length(l, "Error: -d option must be greater than 1");  // raccess.hpp:47-50
   if (params->maximal_span < 1 || params->maximal_span > kWideSpan)
     return fail(PRIB_EINVAL, "maximal span must be in 1.." + std::to_string((int)kWideSpan));
-  if (params->min_accessible_length > kWideSpan)
-    return fail(PRIB_EINVAL, "minimum accessible length must be in 2.." + std::to_string((int)kWideSpan));
+  for (int l = 0; l < n_lengths; l++)
+    if (lengths[l] > kWideSpan)
+      return bad_length(l, "minimum accessible length must be in 2.." + std::to_string((int)kWideSpan));
+  for (int l = 1; l < n_lengths; l++)
+    if (lengths[l] <= lengths[l - 1]) return bad_length(l, "minimum accessible lengths must be strictly increasing");
   if (params->mode < 0 || params->mode > 2)
     return fail(PRIB_EINVAL, "mode must be 0 (auto), 1 (fp64 only) or 2 (exact: reference arithmetic)");
   int ndev = 0;
@@ -1230,7 +1261,8 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   if (!c) return fail(PRIB_ENOMEM, "out of host memory");
   c->prm = *params;
   c->W = params->maximal_span;
-  c->delta = params->min_accessible_length;
+  c->lengths.assign(lengths, lengths + n_lengths);
+  c->evp.assign(PRIB_NUM_PHASES + 1 + 3 * (n_lengths - 1), nullptr);
   const char *pe = getenv("PRIB_PRECISION");
   int fp32_max_span = kFp32MaxSpan;
   if (const char *me = getenv("PRIB_FP32_MAXSPAN")) fp32_max_span = atoi(me);  // tuning knob
@@ -1270,7 +1302,7 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
   if (wide) {
     double klog2 = default_scale_wide().klog2;
     if (const char *e = getenv("PRIB_WIDE_KLOG2")) klog2 = atof(e);  // tuning knob (profiles/scale_scan.py <W> <n> wide)
-    c->wide = wide_create(c->W, c->delta, klog2, err);
+    c->wide = wide_create(c->W, c->lengths, klog2, err);
     if (!c->wide) return bail(fail(PRIB_ECUDA, err));
   }
   if (c->use_fp32) {
@@ -1282,7 +1314,7 @@ int prib_acc_create(prib_ctx **out, const prib_acc_params *params) {
     if (rc != PRIB_OK) return bail(rc == PRIB_EINVAL ? fail(rc, err) : rc);
   }
   if (params->mode == 2 || wide) {
-    c->ex = exact_create(c->W, c->delta, err);
+    c->ex = exact_create(c->W, c->lengths, err);
     if (!c->ex) return bail(fail(PRIB_ECUDA, err));
   }
   const size_t scr64 = (size_t)2 * (c->W + 4) * c->e64.TC * sizeof(double);
@@ -1361,7 +1393,7 @@ int prib_acc_stage(prib_ctx *c, int32_t n, const char *const *seq, const int32_t
     if (layout_columns(len[k]) + 2 * kPad > std::min(max_cols, c->e64.max_cols))
       return fail(PRIB_ECUDA, "sequence " + std::to_string(k) + " does not fit the device DP budget");
   }
-  // packed device output image: [acc L | cond L] per sequence in caller order
+  // packed device output image: [acc L | cond L] per sequence in caller order, one image per length
   std::vector<long long> acc_abs(n), cond_abs(n);
   long long o = 0, total = 0;
   c->seq_len.assign(len, len + n);
@@ -1395,12 +1427,12 @@ int prib_acc_stage(prib_ctx *c, int32_t n, const char *const *seq, const int32_t
     }
     c->h_arena_used = p;
   }
-  if (o > c->out_cap || !c->d_out) {
+  if (c->image_floats() > c->out_cap || !c->d_out) {
     if (c->d_out) cudaFree(c->d_out);
     c->d_out = nullptr;
     c->out_cap = 0;
-    CU(cudaMalloc(&c->d_out, (size_t)std::max<long long>(o, 1) * sizeof(float)));
-    c->out_cap = std::max<long long>(o, 1);
+    CU(cudaMalloc(&c->d_out, (size_t)std::max<long long>(c->image_floats(), 1) * sizeof(float)));
+    c->out_cap = std::max<long long>(c->image_floats(), 1);
   }
   if (c->pipe.on) {
     c->pipe.seq = seq;
@@ -1508,15 +1540,19 @@ int prib_acc_fetch(prib_ctx *c, float *out, const int64_t *acc_off, const int64_
   if (!c->computed) return fail(PRIB_ESTATE, "prib_acc_fetch called before prib_acc_compute");
   CU(cudaSetDevice(c->prm.device));
   // Fast path: the caller's buffer is page-locked (prib_host_alloc / cudaHostRegister) and uses the packed
-  // [acc L | cond L] layout in caller order: the device image is copied straight into it.
-  bool direct = c->out_floats > 0;
+  // [acc L | cond L] layout in caller order, the images of the lengths back to back: the device image is copied
+  // straight into it.
+  const size_t n = c->seq_len.size();
+  const long long total = c->image_floats();
+  bool direct = total > 0;
   {
     long long o = 0;
-    for (size_t k = 0; k < c->seq_len.size() && direct; k++) {
-      const long long L = (long long)c->seq_len[k];
-      direct = acc_off[k] == o && cond_off[k] == o + L;
-      o += 2 * L;
-    }
+    for (size_t l = 0; l < c->lengths.size(); l++)
+      for (size_t k = 0; k < n && direct; k++) {
+        const long long L = (long long)c->seq_len[k];
+        direct = acc_off[l * n + k] == o && cond_off[l * n + k] == o + L;
+        o += 2 * L;
+      }
     if (direct) {
       cudaPointerAttributes at;
       direct = cudaPointerGetAttributes(&at, out) == cudaSuccess && at.type == cudaMemoryTypeHost;
@@ -1525,18 +1561,18 @@ int prib_acc_fetch(prib_ctx *c, float *out, const int64_t *acc_off, const int64_
   }
   float *dst = out;
   if (!direct) {
-    if (c->h_stage_floats < c->out_floats) {
+    if (c->h_stage_floats < total) {
       if (c->h_stage) cudaFreeHost(c->h_stage);
       c->h_stage = nullptr;
       c->h_stage_floats = 0;
-      CU(cudaMallocHost(&c->h_stage, (size_t)c->out_floats * sizeof(float)));
-      c->h_stage_floats = c->out_floats;
+      CU(cudaMallocHost(&c->h_stage, (size_t)total * sizeof(float)));
+      c->h_stage_floats = total;
     }
     dst = c->h_stage;
   }
-  if (c->out_floats > 0) {
+  if (total > 0) {
     CU(cudaEventRecord(c->ev0, c->stream));
-    CU(cudaMemcpyAsync(dst, c->d_out, (size_t)c->out_floats * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(dst, c->d_out, (size_t)total * sizeof(float), cudaMemcpyDeviceToHost, c->stream));
     CU(cudaEventRecord(c->ev1, c->stream));
   }
   CU(cudaMemcpyAsync(c->h_bad, c->d_bad, sizeof(int32_t), cudaMemcpyDeviceToHost, c->stream));
@@ -1545,20 +1581,21 @@ int prib_acc_fetch(prib_ctx *c, float *out, const int64_t *acc_off, const int64_
   if (*c->h_bad != 0)
     return fail(PRIB_ENUMERIC, std::to_string(*c->h_bad) + " accessibility value(s) are not finite: the partition function "
                                "left the double range (span too wide for this sequence); nothing was written");
-  if (c->out_floats > 0) {
+  if (total > 0) {
     float ms = 0;
     CU(cudaEventElapsedTime(&ms, c->ev0, c->ev1));
     c->cnt.d2h_ms += ms;
-    c->cnt.d2h_bytes += c->out_floats * (long long)sizeof(float);
+    c->cnt.d2h_bytes += total * (long long)sizeof(float);
   }
   if (!direct) {
     long long o = 0;
-    for (size_t k = 0; k < c->seq_len.size(); k++) {
-      const size_t L = (size_t)c->seq_len[k];
-      std::memcpy(out + acc_off[k], c->h_stage + o, sizeof(float) * L);
-      std::memcpy(out + cond_off[k], c->h_stage + o + L, sizeof(float) * L);
-      o += 2LL * (long long)L;
-    }
+    for (size_t l = 0; l < c->lengths.size(); l++)
+      for (size_t k = 0; k < n; k++) {
+        const size_t L = (size_t)c->seq_len[k];
+        std::memcpy(out + acc_off[l * n + k], c->h_stage + o, sizeof(float) * L);
+        std::memcpy(out + cond_off[l * n + k], c->h_stage + o + L, sizeof(float) * L);
+        o += 2LL * (long long)L;
+      }
   }
   return PRIB_OK;
 }

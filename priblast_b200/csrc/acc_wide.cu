@@ -101,8 +101,9 @@ int rows_of(int a, int W) { return (a == X_ML || a == X_MR || a == X_MLS || a ==
 }  // namespace
 
 struct WideEngine {
-  int W = 0, delta = 0;
-  KW::SmallTables *d_small = nullptr;
+  int W = 0;
+  std::vector<int> lengths;
+  std::vector<KW::SmallTables *> d_small;  // one per length (they differ in kmul only)
   double *d_int11 = nullptr, *d_int21 = nullptr, *d_int22 = nullptr;
   float *d_log = nullptr;
   double *d_ring = nullptr;  // scan rings, KW::kRing doubles per (sequence, direction); grow-only
@@ -115,7 +116,7 @@ long long wide_state_bytes_per_column(int W) {
   return r * (long long)sizeof(double) + 2 * (long long)sizeof(double);
 }
 
-WideEngine *wide_create(int W, int delta, double klog2, std::string &err) {
+WideEngine *wide_create(int W, const std::vector<int> &lengths, double klog2, std::string &err) {
   std::unique_ptr<HostTablesT<double, kWideSpan>> tab(new (std::nothrow) HostTablesT<double, kWideSpan>());
   if (!tab) {
     err = "out of host memory";
@@ -123,19 +124,29 @@ WideEngine *wide_create(int W, int delta, double klog2, std::string &err) {
   }
   ScaleSpec spec = default_scale_wide();
   spec.klog2 = klog2;
-  if (!build_tables(W, delta, spec, *tab, err)) return nullptr;
   WideEngine *e = new (std::nothrow) WideEngine();
   if (!e) {
     err = "out of host memory";
     return nullptr;
   }
   e->W = W;
-  e->delta = delta;
+  e->lengths = lengths;
   auto up = [&](auto **dst, const auto *src, size_t bytes) {
     return cudaMalloc(dst, bytes) == cudaSuccess && cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice) == cudaSuccess;
   };
-  const bool ok = up(&e->d_small, &tab->small, sizeof(KW::SmallTables)) &&
-                  up(&e->d_int11, tab->e_int11.data(), tab->e_int11.size() * sizeof(double)) &&
+  e->d_small.assign(lengths.size(), nullptr);
+  for (size_t l = 0; l < lengths.size(); ++l) {  // everything uploaded after the loop depends on no delta
+    if (!build_tables(W, lengths[l], spec, *tab, err)) {
+      wide_destroy(e);
+      return nullptr;
+    }
+    if (!up(&e->d_small[l], &tab->small, sizeof(KW::SmallTables))) {
+      err = std::string("wide-span engine tables: ") + cudaGetErrorString(cudaGetLastError());
+      wide_destroy(e);
+      return nullptr;
+    }
+  }
+  const bool ok = up(&e->d_int11, tab->e_int11.data(), tab->e_int11.size() * sizeof(double)) &&
                   up(&e->d_int21, tab->e_int21.data(), tab->e_int21.size() * sizeof(double)) &&
                   up(&e->d_int22, tab->e_int22.data(), tab->e_int22.size() * sizeof(double)) &&
                   up(&e->d_log, tab->log_tbl.data(), tab->log_tbl.size() * sizeof(float));
@@ -149,7 +160,7 @@ WideEngine *wide_create(int W, int delta, double klog2, std::string &err) {
 
 void wide_destroy(WideEngine *e) {
   if (!e) return;
-  cudaFree(e->d_small);
+  for (KW::SmallTables *t : e->d_small) cudaFree(t);
   cudaFree(e->d_int11);
   cudaFree(e->d_int21);
   cudaFree(e->d_int22);
@@ -175,14 +186,14 @@ int wide_run(WideEngine *e, const ExactBatch &b, int32_t *flags, int32_t *bad, c
   memset(&c, 0, sizeof(c));
   c.NC = b.NC;
   c.W = W;
-  c.delta = e->delta;
+  c.delta = e->lengths[0];
   c.rows = W + 4;
   c.nseq = b.n;
   c.S = b.S;
   c.col_seq = b.col_seq;
   c.seq_len = b.seq_len;
   c.seq_off = b.seq_off;
-  c.T = e->d_small;
+  c.T = e->d_small[0];
   c.e_int11 = e->d_int11;
   c.e_int21 = e->d_int21;
   c.e_int22 = e->d_int22;
@@ -217,13 +228,18 @@ int wide_run(WideEngine *e, const ExactBatch &b, int32_t *flags, int32_t *bad, c
   WD_EV(3);
   for (int d = W + 1; d >= kTurn; d--, ++nl) k_wide_outside<<<grid, kWideThreads, 0, st>>>(c, d);
   WD_EV(4);
-  k_wide_strands<<<grid, kWideThreads, 0, st>>>(c);
-  ++nl;
-  WD_EV(5);
-  WD_EV(6);
-  k_wide_finalize<<<grid, kWideThreads, 0, st>>>(c);
-  ++nl;
-  WD_EV(7);
+  for (size_t l = 0; l < e->lengths.size(); ++l) {  // the strand arrays are overwritten from one length to the next
+    c.delta = e->lengths[l];
+    c.T = e->d_small[l];
+    c.out = b.out + (long long)l * b.out_stride;
+    k_wide_strands<<<grid, kWideThreads, 0, st>>>(c);
+    ++nl;
+    WD_EV(5 + 3 * l);
+    WD_EV(6 + 3 * l);
+    k_wide_finalize<<<grid, kWideThreads, 0, st>>>(c);
+    ++nl;
+    WD_EV(7 + 3 * l);
+  }
 #undef WD_EV
   if (launches) *launches = nl;
   return (int)cudaGetLastError();
